@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA path through the C-ABI)
   python bench.py --impl reference --gpus N --steps K ...   the reference's algorithm on the host CPU (oracle port)
+  ... --dump-outputs DIR                                    also write the last timed Solve's Result as DIR/<name>.npy
 
 A "step" is one Solve over one batch of synthetic pods. Workload at N=1: BASELINE.json configs[3], the configuration the
 metric's target is quoted on (C4: 100 000 pods with pod anti-affinity + zone / hostname topology spread x 1 000 instance
@@ -27,6 +28,8 @@ import sys
 import threading
 import time
 from pathlib import Path
+
+import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
@@ -69,6 +72,43 @@ def golden(config, pods, types, seed):
         if g.get("pods") == pods and g.get("types") == types and g.get("seed") == seed:
             return g
     return None
+
+
+DUMP_LIMIT = 64 << 20
+DUMP_OPTION_BYTES = 16 << 20  # C4's full option matrix (20 000 nodes x 1 000 types) is 80 MB: a fixed sample of its rows
+
+
+def dump_outputs(problem, res, out_dir):
+    """Write the Result of the last timed Solve as .npy files, so that two builds can be compared output for output:
+      assign                   [pods] node each pod was placed on, -1 if unschedulable
+      relax_level              [pods] preference relaxation level of each pod
+      new_node_info            [new nodes, 3] provisioner (weight order), pod count, instance-type option count
+      new_node_requests_<res>  [new nodes] summed requests of resource <res>
+      new_node_launch          [new nodes, 2] launched instance type and its price, -1 where the result has no launch choice
+      new_node_options         [rows, instance types] 1 where the type is an option of the node (float32)
+      new_node_options_rows    [rows] which new nodes those rows are: all of them, or a sample fixed by seed 0 when the
+                               full matrix exceeds DUMP_OPTION_BYTES
+    Every other file is float64, which holds these integers and the memory requests (~1e13 milli-bytes) exactly."""
+    nodes = res.to_dict(brief=True)["newNodes"]
+    out = {"assign": res.assign, "relax_level": res.relax_level, "new_node_info": res.new_node_info()}
+    for name in sorted({k for n in nodes for k in n["requests"]}):
+        out[f"new_node_requests_{name}"] = [n["requests"].get(name, 0) for n in nodes]
+    out["new_node_launch"] = np.array([[n["launch"]["type"], n["launch"]["price"]] if "launch" in n else [-1, -1] for n in nodes]).reshape(-1, 2)
+    out = {k: np.asarray(v, dtype=np.float64) for k, v in out.items()}
+    n_types = problem.counts()["instance_types"]
+    rows = min(len(nodes), DUMP_OPTION_BYTES // (4 * n_types))
+    pick = np.sort(np.random.default_rng(0).choice(len(nodes), rows, replace=False))
+    options = np.zeros((rows, n_types), dtype=np.float32)
+    for r, i in enumerate(pick):
+        options[r, res.new_node_options(int(i))] = 1
+    out["new_node_options"] = options
+    out["new_node_options_rows"] = pick.astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit; use a smaller workload")
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(out_dir / f"{name}.npy", a)
 
 
 class ClockSampler:
@@ -174,6 +214,8 @@ def run_reference(args, rank, world):
         "e2e": {"value": value, "unit": "pods/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(problem, res, args.dump_outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -328,6 +370,8 @@ def main():
     ap.add_argument("--types", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU legs and the secondary configurations (profiling runs)")
     ap.add_argument("--no-c5", action="store_true", help="skip the consolidation block (config_c5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the Result of the last timed Solve (rank 0) as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -522,6 +566,8 @@ def main():
             for c in (2, 3):
                 if c != args.config:
                     line[f"config_c{c}"] = secondary(pkg, c)
+        if args.dump_outputs:
+            dump_outputs(problem, res, args.dump_outputs)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()

@@ -1,5 +1,6 @@
 import sys, os
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 from __graft_entry__ import load_pkg
 k=load_pkg()
 p=k.Problem.synth(2,10000,500,42,0)
