@@ -822,7 +822,7 @@ int ksched_upload(ksched_handle* h, const ksched_problem* pb) {
     CUDA_TRY(h, h->d_fd_bound.ensure(nfd * 4)); CUDA_TRY(h, h->d_fd_bound2.ensure(nfd * 4));
   }
   CUDA_TRY(h, h->d_remaining.ensure((size_t)V * KSCHED_MAX_RES));
-  CUDA_TRY(h, h->d_counters.ensure(48));
+  CUDA_TRY(h, h->d_counters.ensure(80));
   {
     size_t need = 0, n2 = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, need, (uint64_t*)nullptr, (uint64_t*)nullptr, (uint32_t*)nullptr, (uint32_t*)nullptr, (int)p1, 0, 64, h->stream);
@@ -1001,7 +1001,7 @@ static int reset_state(ksched_handle* h, const int64_t* d_remaining_src = nullpt
   add(h->d_grp_host.ptr, h->d_grp_host0.ptr, hs * 2);
   if (d_remaining_src)  // simulation on the cluster snapshot: limits with the removed nodes' capacity given back, already on the device
     add(h->d_remaining.ptr, d_remaining_src, (size_t)h->cat.n_templates * KSCHED_MAX_RES * 8);
-  add(h->d_counters.ptr, nullptr, 48 * sizeof(long long));
+  add(h->d_counters.ptr, nullptr, 80 * sizeof(long long));
   add(h->d_fc_state.ptr, nullptr, (size_t)std::max(h->n_classes, 1) * h->cat.n_templates);
   add(h->d_fc_front_state.ptr, nullptr, (size_t)std::max(h->n_classes, 1) * h->cat.n_templates);
   add(h->d_fd_state.ptr, nullptr, (size_t)kFreshMemoSlots);
@@ -1174,6 +1174,13 @@ static void print_pack_profile(const long long* counters) {
   fprintf(stderr, "[pack profile] mask run: build cycles=%lld (refused %lld) loop cycles=%lld pods=%lld entries=%lld\n", counters[38], counters[47], counters[6], counters[7], counters[16]);
   fprintf(stderr, "[pack profile] class_run without mask-key spread: cycles=%lld pods=%lld level+fill iterations=%lld (fill %lld) fresh=%lld per-pod=%lld | with: cycles=%lld pods=%lld fresh=%lld per-pod=%lld\n",
           counters[32], counters[33], counters[34], counters[46], counters[35], counters[44], counters[36], counters[37], counters[39], counters[45]);
+  static const char* kinds[6] = {"round pinned", "round fresh", "round unpinned", "single pinned", "single pin", "single fresh"};
+  for (int k = 0; k < 6; ++k)
+    fprintf(stderr, "[pack profile] mask run %-14s: iterations=%lld pods=%lld cycles=%lld\n", kinds[k], counters[48 + 3 * k], counters[49 + 3 * k],
+            counters[50 + 3 * k]);
+  fprintf(stderr, "[pack profile] mask run declined rounds: na<=1=%lld staged<na=%lld unpinned-first=%lld room-slow=%lld level=%lld no-fresh=%lld "
+                  "unpinned-few=%lld unpinned-pin=%lld\n",
+          counters[66], counters[67], counters[68], counters[69], counters[70], counters[71], counters[72], counters[73]);
 }
 #endif
 
@@ -1181,7 +1188,7 @@ int ksched_download(ksched_handle* h, const ksched_problem* pb, ksched_result* r
   if (!h || !pb || !res || !h->uploaded) return KSCHED_ERR_INVALID;
   CUDA_TRY(h, cudaSetDevice(h->device));
   const int P = h->n_pods, NE = h->n_existing, MAXN = h->max_new, W32 = h->cat.W32, W64 = h->W64, V = h->cat.n_templates;
-  long long counters[48];
+  long long counters[80];
   CUDA_TRY(h, cudaMemcpyAsync(counters, h->d_counters.ptr, sizeof counters, cudaMemcpyDeviceToHost, h->stream));
   CUDA_TRY(h, cudaStreamSynchronize(h->stream));
 #ifdef KSCHED_PROFILE_PACK

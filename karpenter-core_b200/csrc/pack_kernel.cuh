@@ -1383,6 +1383,8 @@ constexpr int kM1Dom = 8;             // domains with ids < kM1Dom; list kM1Dom 
 constexpr int kM1Lists = kM1Dom + 1;
 constexpr int kM1Lv = 12;             // pod counts < kM1Lv
 constexpr uint16_t kM1None = 0xFFFF;
+constexpr int kM1Win = 16;            // lanes kM1Win .. kM1Win + kM1Dom + 1: the first nodes of the unpinned list in a round
+static_assert(kM1Win > kM1Dom && kM1Win + kM1Dom + 1 < 32, "the unpinned window needs its own lanes");
 struct M1Ctx {
   uint16_t tl[kM1Lv][kM1Lists];       // last node of the bucket (kM1None: empty)
   uint16_t head[kM1Lists];            // first node of the list (between two entries of the warp loop)
@@ -1863,7 +1865,21 @@ __device__ __noinline__ void class_run(const PodRegs& first_in) {
         // count + self - min <= maxSkew as count - min <= slack in 32 bits: counts are pod counts (< 2^30), so a slack of 2^30
         // or more admits every domain exactly like the 64-bit form of the per-pod loop
         const int slack = m_bias0 < -(1 << 30) ? (1 << 30) : -m_bias0;
+#ifdef KSCHED_PROFILE_PACK
+        // iterations by kind (k: 0 round of pinned heads, 1 round with fresh nodes, 2 round that pins unpinned nodes, 3 single
+        // step on a pinned head, 4 single step that pins an unpinned node, 5 single fresh node): count, pods, cycles
+#define M1_KIND(k, pods) { if (L == 0) { s.counters[48 + 3 * (k)] += 1; s.counters[49 + 3 * (k)] += (pods); s.counters[50 + 3 * (k)] += clock64() - it_t0; } }
+        // declined rounds (r: 0 na <= 1, 1 too few staged entries, 2 unpinned head first, 3 room kRoomSlow, 4 count + 1 >= kM1Lv,
+        // 5 no fresh node possible, 6 unpinned round: too few candidates, 7 unpinned round: a pin precondition fails)
+#define M1_DECLINE(r) { if (L == 0) s.counters[66 + (r)] += 1; }
+#else
+#define M1_KIND(k, pods) {}
+#define M1_DECLINE(r) {}
+#endif
         while (li < i_end) {
+#ifdef KSCHED_PROFILE_PACK
+          const long long it_t0 = clock64();
+#endif
           const int mn = __reduce_min_sync(FULL, valid ? cnt_d : INT32_MAX);
           const bool allowed = valid && cnt_d - mn <= slack;
           const unsigned okm = __ballot_sync(FULL, allowed);
@@ -1980,9 +1996,136 @@ __device__ __noinline__ void class_run(const PodRegs& first_in) {
                 ltick += na;
                 li += na;
                 __syncwarp();
+                M1_KIND(nf ? 1 : 0, na)
                 continue;
               }
-            }
+              if (ukey != ~0ull && !(hv == okm && ukey > mx)) {
+                // an unpinned node comes before some head (or a domain has no head): the one-pod steps of the round, replayed
+                // in key order over the candidates - the heads of the admissible lists and the first na unpinned nodes. A
+                // head takes a pod while its domain is still open in the round; an unpinned node takes one and is pinned to
+                // the lowest open domain id (run_pick). The window walks one node further than the round can take, so the
+                // unpinned list's next head and the node behind it are known without another load.
+                const int u0 = __shfl_sync(FULL, h, kM1Dom), u1 = __shfl_sync(FULL, n1, kM1Dom);
+                int us = L == kM1Win ? u0 : (L == kM1Win + 1 ? u1 : -1);  // lane kM1Win + j: the j-th node of the unpinned list
+                int cur = u1;
+                for (int j = 2; j <= na + 1; ++j) {
+                  cur = cur >= 0 ? nxt_of(cur) : -1;
+                  if (L == kM1Win + j) us = cur;
+                }
+                unsigned long long uk = ~0ull;
+                uint32_t ur = 0;
+                if (us >= 0) { uk = hs->key[us]; ur = rpv[us]; }
+                const bool un = L >= kM1Win && L < kM1Win + na && us >= 0;
+                const bool cnd = hd || un;
+                const unsigned long long ck = hd ? hk : uk;
+                const unsigned cm = __ballot_sync(FULL, cnd);
+                int pos = 0;  // position among the candidates
+                for (unsigned m = cm; m; m &= m - 1) pos += __shfl_sync(FULL, ck, __ffs(m) - 1) < ck;
+                // 4 bits per position: the head's domain, or 8 for an unpinned node (those come in list order)
+                const unsigned long long code = cnd ? (unsigned long long)(un ? 8 : L) << (4 * pos) : 0ull;
+                const unsigned long long desc = ((unsigned long long)__reduce_or_sync(FULL, (unsigned)(code >> 32)) << 32) |
+                                                __reduce_or_sync(FULL, (unsigned)code);
+                unsigned open = okm;
+                unsigned long long asg = 0;  // one byte per domain: 0x80 gets a pod | 0x40 from unpinned node j << 3 | position
+                int ju = 0;                  // unpinned nodes the round takes
+                for (int p = 0, nc = __popc(cm); p < nc && open; ++p) {
+                  const int cd = (int)(desc >> (4 * p)) & 15;
+                  const int d = cd == 8 ? __ffs(open) - 1 : cd;
+                  if ((open >> d) & 1) {
+                    asg |= (unsigned long long)(0x80 | (cd == 8 ? 0x40 | ju << 3 : 0) | (na - __popc(open))) << (8 * d);
+                    open &= ~(1u << d);
+                  }
+                  ju += cd == 8;
+                }
+                const unsigned b = L < kM1Dom ? (unsigned)(asg >> (8 * L)) & 0xFF : 0u;
+                const int src = (b & 0x40) ? kM1Win + ((b >> 3) & 7) : L;
+                const int ua = __shfl_sync(FULL, us, src);
+                const unsigned long long uka = __shfl_sync(FULL, uk, src);
+                const uint32_t ura = __shfl_sync(FULL, ur, src);
+                // this lane's pod goes to node a (room word rp2's source, count c) at position rank of the round: its own
+                // head, or with `pin` the unpinned node the commit pins to this domain
+                const bool mine = (b & 0x80) != 0, pin = (b & 0x40) != 0;
+                const int rank = b & 7, a = pin ? ua : h;
+                const uint32_t rp = pin ? ura : hr;
+                const int c = (int)((pin ? uka : hk) >> 32);
+                bool bad_m = mine && ((rp & 0xFFFF) == kRoomSlow || c + 1 >= kM1Lv);
+                if (pin) bad_m = bad_m || !((rc.m_neutral[0] >> L) & 1) || !((zv[a] & (1u << 17)) || rc.m_wk[0]);
+#ifdef KSCHED_PROFILE_PACK
+                if (open) M1_DECLINE(6)
+                else if (__any_sync(FULL, bad_m)) M1_DECLINE(7)
+#endif
+                // a domain left open needs a fresh node, and these are only replayed when no unpinned node is left
+                if (open == 0 && !__any_sync(FULL, bad_m)) {
+                  bool closed_l = false;
+                  if (mine) {
+                    const int mytick = ltick + rank;
+                    if (!pin) pop_head(c);
+                    uint32_t rp2 = rp - 1 + (1u << 16);
+                    for (int j = 0; j < n_host; ++j) {  // Topology.Record, hostname groups
+                      const int times = rc.h_times[j];
+                      const int old = hc[j * kTopoCap + a];
+                      const int now = old + times > 0xFFFF ? 0xFFFF : old + times;
+                      if (times) hc[j * kTopoCap + a] = (uint16_t)now;
+                      if (now > rc.h_lim[j]) rp2 |= kRpDead;
+                    }
+                    const unsigned long long nkey = order_key(c + 1, -(mytick + 1));
+                    unsigned long long skey = nkey;
+                    rc.q_node[buf][li + rank] = -(a + 2);
+                    if (pin) {  // requirements.Add(In{L}) on the node, as the one-pod step does it
+                      const int n = hs->node[a], k = rc.m_key[0];
+                      zv[a] = (1u << L) | (3u << 16);
+                      s.nn_vals[(size_t)k * MAXN + n] = 1ull << L;
+                      atomicOr(reinterpret_cast<unsigned long long*>(&s.nn_meta[n]), 1ull << (KSCHED_META_PRESENT_SHIFT + k));
+                      atomicAnd(reinterpret_cast<unsigned long long*>(&s.nn_meta[n]), ~(1ull << (KSCHED_META_COMPLEMENT_SHIFT + k)));
+                    }
+                    if ((rp2 & 0xFFFF) == 0) {  // the class no longer fits by resources: does anything? (node_closed)
+                      const int placed = (rp2 >> 16) & 0x7FFF;
+                      long long nq[kHotRes], cb1[kHotRes], cb2[kHotRes];
+#pragma unroll
+                      for (int r = 0; r < kHotRes; ++r) { nq[r] = hs->q[r][a] + placed * p_req[r]; cb1[r] = hs->bound[r][a]; cb2[r] = hs->bound2[r][a]; }
+                      const unsigned short fl = (unsigned short)(hs->flags[a] | ((p_res & 0xF) << 1));
+                      if (node_closed(nq, min_req, RH, cb1, cb2, fl)) {
+                        skey = ~0ull;
+                        hs->nn_last[a] = ((unsigned long long)(unsigned)(c + 1) << 32) | (unsigned)(-(mytick + 1));
+                        closed_l = true;
+                      }
+                    }
+                    hs->key[a] = skey;
+                    rpv[a] = rp2;
+                    // (a pinned node enters a list whose own head is not placed in this round: lane L stays its only writer)
+                    if ((rp2 & 0xFFFF) != 0 && !(rp2 & kRpDead)) insert_front(a, c + 1, nkey, rp2);
+                    ++cnt_d;
+                  }
+                  // the unpinned list loses its first ju nodes; a bucket they emptied has no tail any more
+                  const int nh = __shfl_sync(FULL, us, kM1Win + ju), nn = __shfl_sync(FULL, us, kM1Win + ju + 1);
+                  const unsigned long long nhk = __shfl_sync(FULL, uk, kM1Win + ju), nnk = __shfl_sync(FULL, uk, kM1Win + ju + 1);
+                  const uint32_t nhr = __shfl_sync(FULL, ur, kM1Win + ju), nnr = __shfl_sync(FULL, ur, kM1Win + ju + 1);
+                  const unsigned long long uk_nx = __shfl_down_sync(FULL, uk, 1);
+                  const bool emptied = L >= kM1Win && L < kM1Win + ju && (uk_nx >> 32) != (uk >> 32);
+                  if (emptied) m1.tl[(int)(uk >> 32)][kM1Dom] = kM1None;
+                  const bool any_emptied = __any_sync(FULL, emptied);
+                  if (L == kM1Dom) { h = nh; hk = nhk; hr = nhr; n1 = nn; nk = nnk; nr = nnr; }
+                  if (any_emptied) {
+                    __syncwarp();
+                    if (L == kM1Dom) level_state();
+                  }
+                  const unsigned tb = __ballot_sync(FULL, closed_l);
+                  if (L == 0 && tb) rc.tomb = rc.tomb + __popc(tb);
+                  ltick += na;
+                  li += na;
+                  __syncwarp();
+                  M1_KIND(2, na)
+                  continue;
+                }
+              }
+#ifdef KSCHED_PROFILE_PACK
+              else if (ukey != ~0ull && hv != 0 && ukey <= mx) M1_DECLINE(2)
+              else if (__any_sync(FULL, bad_l && (hr & 0xFFFF) == kRoomSlow)) M1_DECLINE(3)
+              else if (__any_sync(FULL, bad_l)) M1_DECLINE(4)
+              else M1_DECLINE(5)
+#endif
+            } else if (na <= 1) M1_DECLINE(0)
+            else M1_DECLINE(1)
           }
           if (wkey != ~0ull) {
             const int wl = __ffs(__ballot_sync(FULL, key == wkey)) - 1;
@@ -2044,6 +2187,7 @@ __device__ __noinline__ void class_run(const PodRegs& first_in) {
             ++ltick;
             ++li;
             __syncwarp();  // lane 0's key / room words before a later pop fetches them
+            M1_KIND(pin ? 4 : 3, 1)
             if (reason == 2) break;
           } else {
             // ---- nobody accepts: NewNode + Add replayed from the variant of the domain a fresh node gets
@@ -2089,8 +2233,11 @@ __device__ __noinline__ void class_run(const PodRegs& first_in) {
             }
             ++ltick; ++lnew; ++lact; ++li;
             __syncwarp();
+            M1_KIND(5, 1)
           }
         }
+#undef M1_KIND
+#undef M1_DECLINE
         __syncwarp();
         // every warp's copy of the spread counters follows (the per-pod loop and the write-back read them)
         if (L < kM1Dom) for (int w = 0; w < nwarps; ++w) rc.cnt[w][0][L] = cnt_d;
